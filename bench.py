@@ -2,7 +2,7 @@
 """bench.py - headline benchmark: train patches/sec of the 64x64 SR CondVAE step on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--workload cond_grid|cond_grid1024|vae|cond256|sample]
+                    [--workload cond_grid|cond_grid1024|vae|cond256|sample] [--dump-outputs DIR]
 
 Default workload at every N (weak scaling): BASELINE.json config 3 - CondVAE cr=2, P=64, grid mode: 8 synthetic 256x256
 multispectral tiles per GPU -> 128 patches per GPU (64 tiles / 1024 patches at N=8), bf16 compute, fp32 master
@@ -17,6 +17,11 @@ of the loss inside the timed region.  `--impl reference` times the CPU restateme
 host cores on a bounded sample of the same workload (same per-step batch).  Outside the timed regions the default line
 also carries `roofline` (dominant kernel), `roofline_hbm` (the bandwidth-bound kernels at the bench batch),
 `cpu_baseline`, `gpu_reference` (the reference's torch ops under cuDNN on the same GPU) and, for N > 1, `ddp_check`.
+
+`--dump-outputs DIR` writes what the last step of the device-timed region computed, as DIR/<name>.npy (rank 0):
+`loss_terms` (the tensor the step returns), `gammas` and `params_sample` (the updated weights: a fixed PCG64 sample of
+the fp32 parameter store) for the training workloads, `std` (the posterior std maps) for `sample`.  Inputs, weights and
+noise are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +39,7 @@ for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 # ---- workloads (BASELINE.json configs 2-5).  flop = algorithmic FLOPs per unit of one optimisation step / sample
@@ -56,6 +62,24 @@ WORKLOADS = {
                    name="CondVAE cr=2 P=64 inference: 1 LR tile -> 16 patches x 32 posterior samples per step (config 5)"),
 }
 SAMPLES_PER_PATCH = 32
+DUMP_PARAMS = 1 << 22       # weights written by --dump-outputs: 16 MB of fp32, well inside the dump's 64 MB
+
+
+def timed_step_outputs(out, tr):
+    """Host copies of what the last timed step computed: the step's return value and, for a training step (`tr` given),
+    the loss weights and a fixed sample of the updated fp32 parameter store."""
+    def host(t):
+        a = t.detach().cpu()
+        return (a if a.dtype in (torch.float32, torch.float64) else a.float()).numpy()
+
+    if tr is None:
+        return {"std": host(out)}
+    flat = tr.rt.store.flat
+    if flat.numel() > DUMP_PARAMS:
+        # numpy's PCG64 draws the same indices on every host
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_PARAMS, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    return {"loss_terms": host(out), "gammas": host(tr.gam[:tr.n_gammas]), "params_sample": host(flat)}
 
 
 def peaks():
@@ -335,7 +359,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -456,6 +483,8 @@ def main():
         barrier()
     ms = e0.elapsed_time(e1)
     launches = rt.launches - l0
+    # taken before the e2e region steps the model on
+    dump = timed_step_outputs(out, None if is_sample else tr) if args.dump_outputs and rank == 0 else None
     out_small = out if out.numel() <= 8 else out.flatten()[:5]
     last_loss = float(out_small.flatten()[-1])
 
@@ -558,6 +587,10 @@ def main():
         }
         if ddp is not None:
             line["ddp_check"] = ddp
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         # Leave without tearing NCCL down: communicators captured inside CUDA graphs make destroy_process_group() hang

@@ -25,6 +25,12 @@ def test_reference_arm_prints_contract_line():
     assert e2e["value"] == d["value"] and e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0
 
 
+def test_steps_below_one_is_rejected():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                       capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
 def test_reference_arm_non_zero_ranks_exit_quietly():
     """Under torchrun (N > 1) only rank 0 runs the CPU arm; the other ranks exit 0 without output."""
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT="29599")
