@@ -319,6 +319,21 @@ int svrs_sample_tail_stats(const void* x, int dtype, const void* w_kn, const flo
                            float* mean_nchw, float* std_map, float* mae_map, float* mse_map, float* bias_map,
                            float* sample0_nchw, void* stream);
 
+/* ---- SSIM metrics of evaluate(): Metrics/SSIM_LR, SSIM_HR, SSIM_SR of Cond_SRVAE (cond_vae.py:387-525) and Metrics/SSIM of
+ *      VAE (vae.py:142-216), which the reference computes with
+ *      skimage.metrics.structural_similarity(a, b, win_size=11, data_range=1.0, channel_axis=0)   (csrc/ssim.cu).
+ * svrs_ssim: a, b fp32 NCHW contiguous [N][C][H][W]; out[n] (double) = that value for the pair (a[n], b[n]) with scikit-image's
+ *      defaults (uniform win x win window, sample covariance win^2/(win^2-1), C1 = (0.01 R)^2, C2 = (0.03 R)^2, R = data_range):
+ *      the mean of the SSIM map over the (H-win+1) x (W-win+1) interior positions of each plane, averaged over the C planes.
+ *      win odd, 3 <= win <= min(H, W).  Shared-memory staging of full-width bands limits the width:
+ *      4 * W * (2 * (15 + win) + 90) <= 227 KB, i.e. W <= 409 at win = 11.  N == 0 enqueues nothing.
+ *      workspace: svrs_ssim_workspace_doubles(N, C, H, W, win) doubles (one partial per band of 16 output rows of a plane),
+ *      no initialisation needed.  Two launches, no atomics: repeated calls give bitwise-identical results.
+ * svrs_ssim_workspace_doubles returns -1 (with svrs_last_error) for arguments svrs_ssim rejects. */
+int64_t svrs_ssim_workspace_doubles(int N, int C, int H, int W, int win);
+int svrs_ssim(const float* a, const float* b, int N, int C, int H, int W, int win, float data_range, double* workspace,
+              double* out, void* stream);
+
 /* ---- backward of the fused epilogue activations from their OUTPUT y:
  *      sigmoid: dx = dy*y*(1-y) ; hardtanh(-7,7): dx = dy if -7 < y < 7 else 0.  In-place (dx == dy) allowed. */
 int svrs_act_bwd(const void* y, const void* dy, void* dx, int dtype, int act, int64_t n, void* stream);

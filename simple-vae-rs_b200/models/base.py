@@ -60,12 +60,6 @@ class BaseVAE(nn.Module, metaclass=abc.ABCMeta):
         self.patch_size: int = patch_size
         self.callbacks: List[Callback] = [] if callbacks is None else callbacks
         self.num_params: int = 0
-        # SSIM / LPIPS metrics of evaluate() are out of the hot-path scope; used only if installed.
-        try:
-            from skimage import metrics as _skm
-            self.ssim = _skm.structural_similarity
-        except Exception:
-            self.ssim = None
         self.lpips_fn = None
         self._eng = None
         self._trainer = None

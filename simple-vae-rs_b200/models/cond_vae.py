@@ -218,31 +218,33 @@ class Cond_SRVAE(BaseVAE):
 
     # ------------------------------------------------------------------ epoch-rate hooks
     def evaluate(self, val_loader, wandb_run, epoch, full_val=False):
-        """cond_vae.py:387-525.  SSIM / LPIPS need scikit-image / lpips (third-party, CPU, epoch-rate; outside
-        the hot-path scope): they are computed only when those packages are installed.  Image logging keeps
-        the reference's keys."""
+        """cond_vae.py:387-525.  On full-validation epochs the SSIM metrics (skimage's structural_similarity with
+        win_size=11, data_range=1.0, averaged over the validation images) are computed on the device (svrs_native.metrics);
+        SSIM_LR is not logged when the LR patches are smaller than the window (patch_size < 22).  LPIPS needs pretrained
+        AlexNet weights and is not computed.  Image logging keeps the reference's keys."""
+        from svrs_native import metrics
         device = next(self.parameters()).device
         batch = next(iter(val_loader))
         y, x = [t.to(device) for t in batch]
         with torch.no_grad():
             x_hat, y_hat, *_ = self.forward(x, y)
             x_sr = self.conditional_generation(y)
-        if full_val and self.ssim is not None:
-            tot = {"ssim_y": 0.0, "ssim_x": 0.0, "ssim_sr": 0.0}
+        keys = [k for k, img in (("Metrics/SSIM_LR", y), ("Metrics/SSIM_HR", x), ("Metrics/SSIM_SR", x))
+                if min(img.shape[-2:]) >= 11]
+        if full_val and keys:
+            tot = {k: torch.zeros((), device=device, dtype=torch.float64) for k in keys}
             cnt = 0
             for b in val_loader:
                 yy, xx = [t.to(device) for t in b]
                 with torch.no_grad():
                     xh, yh, *_ = self.forward(xx, yy)
                     sr = self.conditional_generation(yy)
-                for oy, ry, ox, rx, gen in zip(yy, yh, xx, xh, sr):
-                    kw = dict(win_size=11, data_range=1.0, channel_axis=0)
-                    tot["ssim_y"] += self.ssim(oy.cpu().numpy(), ry.cpu().numpy(), **kw)
-                    tot["ssim_x"] += self.ssim(ox.cpu().numpy(), rx.cpu().numpy(), **kw)
-                    tot["ssim_sr"] += self.ssim(ox.cpu().numpy(), gen.cpu().numpy(), **kw)
+                pairs = {"Metrics/SSIM_LR": (yy, yh), "Metrics/SSIM_HR": (xx, xh), "Metrics/SSIM_SR": (xx, sr)}
+                for k in keys:
+                    tot[k] += metrics.ssim(*pairs[k]).sum()
                 cnt += yy.size(0)
-            wandb_run.log({"Metrics/SSIM_LR": tot["ssim_y"] / cnt, "Metrics/SSIM_HR": tot["ssim_x"] / cnt,
-                           "Metrics/SSIM_SR": tot["ssim_sr"] / cnt}, step=epoch)
+            vals = torch.stack([tot[k] for k in keys]).tolist()         # one host read for all metrics
+            wandb_run.log({k: v / cnt for k, v in zip(keys, vals)}, step=epoch)
         if epoch % 10 == 0 or epoch == 1:
             imgs = {"Images/LR_Input": y[:4], "Images/HR_Input": x[:4], "Images/LR_Recon": y_hat[:4],
                     "Images/HR_Recon": x_hat[:4], "Images/SR_Output": x_sr[:4]}
@@ -254,7 +256,8 @@ class Cond_SRVAE(BaseVAE):
 
     def on_train_start(self, **kwargs):
         """cond_vae.py:527-582: the gammas join the optimizer as a second param group (same lr, unclipped).
-        The bicubic SSIM/LPIPS baseline of the reference needs lpips/skimage and is skipped without them."""
+        The bicubic SSIM/LPIPS baseline of the reference is not computed (LPIPS needs pretrained AlexNet weights); a cached
+        baseline_ckpt.pth is loaded."""
         self.gammax.requires_grad = True
         self.gammay.requires_grad = True
         have = {id(p) for g in self.optimizer.param_groups for p in g["params"]}

@@ -112,22 +112,24 @@ class VAE(BaseVAE):
         return loss, {"Loss/val_loss": loss, "Loss/val_mse": mse, "Loss/val_kld": kld}
 
     def evaluate(self, val_loader, wandb_run, epoch, full_val=False):
-        """vae.py:142-216: SSIM needs scikit-image (optional, outside the hot-path scope); image logging kept."""
+        """vae.py:142-216: on full-validation epochs Metrics/SSIM (skimage's structural_similarity with win_size=11,
+        data_range=1.0, averaged over the validation images) is computed on the device (svrs_native.metrics); it is not
+        logged for patches smaller than the window.  Image logging kept."""
+        from svrs_native import metrics
         device = next(self.parameters()).device
         x, _ = next(iter(val_loader))
         x = x.to(device)
         with torch.no_grad():
             x_hat, _, _ = self.forward(x)
-        if full_val and self.ssim is not None:
-            tot, cnt = 0.0, 0
+        if full_val and min(x.shape[-2:]) >= 11:
+            tot, cnt = torch.zeros((), device=device, dtype=torch.float64), 0
             for b, _ in val_loader:
                 b = b.to(device)
                 with torch.no_grad():
                     r, _, _ = self.forward(b)
-                for o, rr in zip(b, r):
-                    tot += self.ssim(o.cpu().numpy(), rr.cpu().numpy(), win_size=11, data_range=1.0, channel_axis=0)
+                tot += metrics.ssim(b, r).sum()
                 cnt += b.size(0)
-            wandb_run.log({"Metrics/SSIM": tot / cnt}, step=epoch)
+            wandb_run.log({"Metrics/SSIM": float(tot) / cnt}, step=epoch)
         if epoch % 5 == 0 or epoch == 1:
             try:
                 wandb_run.log({"Images/Input": [wandb.Image(i.permute(1, 2, 0).cpu().numpy()) for i in x[:4]]}, step=epoch)
