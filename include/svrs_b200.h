@@ -210,7 +210,9 @@ int svrs_philox_normal(float* out, int B, int Wd, uint64_t seed, uint32_t stream
  * finalize turns them into the reference's terms out[5] = {mse_x, kld_u, mse_y, kld_z, their sum} (fp32):
  *   mse = ssq/(2 g^2) + n log g ;  kld = 0.5 * sum / B.   Unused pieces: pass NULL / n = 0.
  * dt_x / dt_y are the dtypes of the reconstructions, dt_tx / dt_ty those of the targets (the fused step keeps the
- * targets in fp32 NHWC next to the bf16 conv operands; any layout works as long as recon and target share it). */
+ * targets in fp32 NHWC next to the bf16 conv operands; any layout works as long as recon and target share it).
+ * Requirements (else SVRS_E_ARG, nothing enqueued): every pointer 16-byte aligned; with mu1 given, lv1 too, W1 > 0 and
+ * ld1 >= W1; with mu2 given, lv2 / mu3 / lv3 too, W2 > 0 and ld2, ld3 >= W2; all widths and strides multiples of 4. */
 int svrs_elbo_fwd(const void* recon_x, const void* x, int dt_x, int dt_tx, int64_t n_x,
                   const void* recon_y, const void* y, int dt_y, int dt_ty, int64_t n_y,
                   const float* mu1, const float* lv1, int64_t ld1, int W1,
@@ -224,7 +226,8 @@ int svrs_elbo_finalize(const double* acc, int64_t n_x, int64_t n_y, int B, const
  * d_mu1 = g*mu1/B ; d_lv1 = g*0.5*(exp(lv1)-1)/B
  * d_mu2 = g*(mu2-mu3)exp(-lv3)/B = -d_mu3 ; d_lv2 = g*0.5*(exp(lv2-lv3)-1)/B
  * d_lv3 = g*0.5*(1 - exp(lv2-lv3) - (mu2-mu3)^2 exp(-lv3))/B
- * latent grads are written with the same row strides as their inputs (dst strides dld1/dld2/dld3).
+ * latent grads are written with their own row strides dld1/dld2/dld3: multiples of 4, and >= W1 / W2 / W2 whenever an
+ * output of that pair is given; the input requirements of svrs_elbo_fwd apply.
  * dt_dx / dt_dy: dtype of d_recon_x / d_recon_y.  act = SVRS_ACT_SIGMOID: the reconstructions are sigmoid outputs and
  * d_recon_* receives the gradient wrt the PRE-activation, d * r * (1 - r) (nn.Sigmoid backward folded in); else SVRS_ACT_NONE. */
 int svrs_elbo_bwd(const void* recon_x, const void* x, int dt_x, int dt_tx, int64_t n_x, void* d_recon_x, int dt_dx,
@@ -294,7 +297,8 @@ int svrs_patch_gather_normalize(const void* tiles, int src_is_i16, int T, int C,
  *   written together with y_to_z(y) as the decoder_x input rows (torch.cat((y_enc, z), dim=1), cond_vae.py:272):
  *      stack[(b*S + s)][0:Wz] = yflat[b][0:Wz] ; stack[(b*S + s)][Wz:2Wz] = z(b, s)        (fp32, NCHW-flat order)
  *   mu3 / lv3 rows have stride ld3, yflat rows stride ldy.  eps [B*S][Wz] fp32 or NULL = on-device Philox4x32-10 with the
- *   counter layout of svrs_reparam_fwd (row = sample_offset + b*S + s). */
+ *   counter layout of svrs_reparam_fwd (row = sample_offset + b*S + s).  Requires Wz, ld3, ldy multiples of 4,
+ *   ld3 >= Wz, ldy >= Wz and 16-byte aligned mu3 / lv3 / yflat / eps / stack (else SVRS_E_ARG, nothing enqueued). */
 int svrs_sample_latents(const float* mu3, const float* lv3, int64_t ld3, const float* yflat, int64_t ldy,
                         const float* eps, float* stack, int B, int S, int Wz, uint64_t seed, int stream_id,
                         uint64_t sample_offset, const int64_t* step_ptr, void* stream);
@@ -310,8 +314,8 @@ int svrs_sample_latents(const float* mu3, const float* lv3, int64_t ld3, const f
  *      sample0_nchw [B][4][H][W] = samples[0]                                          (base.py:318)
  * w_kn = p10 pack [9][16][4] of the layer (dtype), bias fp32[4] or NULL, target_nhwc fp32 [B][H][W][4] or NULL (then only
  * mean / std / sample0 are produced).  Every output pointer may be NULL.  splits in [1, S] (svrs_sample_tail_splits gives
- * the default); scratch = svrs_sample_tail_scratch_floats(B, H, W, splits) floats.  Returns SVRS_E_UNSUPPORTED unless
- * (Cin, Cout) == (16, 4). */
+ * the default); scratch = svrs_sample_tail_scratch_floats(B, H, W, splits) floats.  x and target_nhwc must be 16-byte
+ * aligned (else SVRS_E_ARG).  Returns SVRS_E_UNSUPPORTED unless (Cin, Cout) == (16, 4). */
 int svrs_sample_tail_splits(int B, int S, int H, int W);
 int64_t svrs_sample_tail_scratch_floats(int B, int H, int W, int splits);
 int svrs_sample_tail_stats(const void* x, int dtype, const void* w_kn, const float* bias, const float* target_nhwc,

@@ -59,6 +59,9 @@ static inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
 }
 #define SVRS_LAUNCH(kernel, grid, block, smem, st, ...) svrs::launch_k(kernel, dim3(grid), dim3(block), (size_t)(smem), st, __VA_ARGS__)
 
+// NULL or 16-byte aligned: the condition for the float4 / uint4 accesses of the streaming kernels
+static inline bool al16(const void* p) { return p == nullptr || ((uintptr_t)p & 15) == 0; }
+
 static inline int num_sms() {
     static int n = 0;
     if (n == 0) {

@@ -265,17 +265,21 @@ __global__ void __launch_bounds__(256) elbo_bwd_kernel(const __grid_constant__ E
         nll_bwd_segment(f.ry, f.dty, f.y, f.dtty, a.dry, a.dtdy, f.ny, c, a.act, gtid, gsize);
     }
     const float invB = 1.0f / (float)f.B;
-    if (f.mu1 && a.dmu1 && a.dlv1) {
+    if (f.mu1 && (a.dmu1 || a.dlv1)) {
         const int wq = f.W1 / 4;
         const long long nvec = (long long)f.B * wq;
         const float k = g_klu * invB;
         for (long long i = gtid; i < nvec; i += gsize) {
             long long r = i / wq, c = (i % wq) * 4;
-            float4 m = *reinterpret_cast<const float4*>(f.mu1 + r * f.ld1 + c);
-            float4 l = *reinterpret_cast<const float4*>(f.lv1 + r * f.ld1 + c);
-            *reinterpret_cast<float4*>(a.dmu1 + r * a.dld1 + c) = make_float4(k * m.x, k * m.y, k * m.z, k * m.w);
-            *reinterpret_cast<float4*>(a.dlv1 + r * a.dld1 + c) =
-                make_float4(k * 0.5f * (expf(l.x) - 1.f), k * 0.5f * (expf(l.y) - 1.f), k * 0.5f * (expf(l.z) - 1.f), k * 0.5f * (expf(l.w) - 1.f));
+            if (a.dmu1) {
+                float4 m = *reinterpret_cast<const float4*>(f.mu1 + r * f.ld1 + c);
+                *reinterpret_cast<float4*>(a.dmu1 + r * a.dld1 + c) = make_float4(k * m.x, k * m.y, k * m.z, k * m.w);
+            }
+            if (a.dlv1) {
+                float4 l = *reinterpret_cast<const float4*>(f.lv1 + r * f.ld1 + c);
+                *reinterpret_cast<float4*>(a.dlv1 + r * a.dld1 + c) =
+                    make_float4(k * 0.5f * (expf(l.x) - 1.f), k * 0.5f * (expf(l.y) - 1.f), k * 0.5f * (expf(l.z) - 1.f), k * 0.5f * (expf(l.w) - 1.f));
+            }
         }
     }
     if (f.mu2) {
@@ -314,8 +318,6 @@ static unsigned ew_grid2(long long nvec) {
     if (b < 1) b = 1;
     return (unsigned)b;
 }
-
-static bool al16(const void* p) { return p == nullptr || ((uintptr_t)p & 15) == 0; }
 
 }  // namespace svrs
 
@@ -358,9 +360,15 @@ static int fill_elbo_args(ElboArgs& a, const void* recon_x, const void* x, int d
     SVRS_CHECK_ARG((dt_x == SVRS_F32 || dt_x == SVRS_BF16) && (dt_y == SVRS_F32 || dt_y == SVRS_BF16) &&
                    (dt_tx == SVRS_F32 || dt_tx == SVRS_BF16) && (dt_ty == SVRS_F32 || dt_ty == SVRS_BF16), "elbo: bad dtype");
     SVRS_CHECK_ARG(al16(recon_x) && al16(x) && al16(recon_y) && al16(y), "elbo: image pointers must be 16B aligned");
-    if (mu1) SVRS_CHECK_ARG(lv1 && W1 % 4 == 0 && ld1 % 4 == 0 && al16(mu1) && al16(lv1), "elbo: kl1 needs W1,ld1 %% 4 == 0 and 16B alignment");
-    if (mu2) SVRS_CHECK_ARG(lv2 && mu3 && lv3 && W2 % 4 == 0 && ld2 % 4 == 0 && ld3 % 4 == 0 && al16(mu2) && al16(lv2) && al16(mu3) && al16(lv3),
-                            "elbo: kl23 needs W2,ld2,ld3 %% 4 == 0 and 16B alignment");
+    if (mu1) {
+        SVRS_CHECK_ARG(lv1 && W1 > 0 && W1 % 4 == 0 && ld1 % 4 == 0 && al16(mu1) && al16(lv1), "elbo: kl1 needs W1 > 0, W1,ld1 %% 4 == 0 and 16B alignment");
+        SVRS_CHECK_ARG(ld1 >= W1, "elbo: kl1 row stride ld1 (%lld) < W1 (%d)", (long long)ld1, W1);
+    }
+    if (mu2) {
+        SVRS_CHECK_ARG(lv2 && mu3 && lv3 && W2 > 0 && W2 % 4 == 0 && ld2 % 4 == 0 && ld3 % 4 == 0 && al16(mu2) && al16(lv2) && al16(mu3) && al16(lv3),
+                       "elbo: kl23 needs W2 > 0, W2,ld2,ld3 %% 4 == 0 and 16B alignment");
+        SVRS_CHECK_ARG(ld2 >= W2 && ld3 >= W2, "elbo: kl23 row strides ld2 (%lld) / ld3 (%lld) < W2 (%d)", (long long)ld2, (long long)ld3, W2);
+    }
     a.rx = recon_x; a.x = x; a.ry = recon_y; a.y = y; a.dtx = dt_x; a.dty = dt_y; a.dttx = dt_tx; a.dtty = dt_ty; a.nx = n_x; a.ny = n_y;
     a.mu1 = mu1; a.lv1 = lv1; a.mu2 = mu2; a.lv2 = lv2; a.mu3 = mu3; a.lv3 = lv3;
     a.ld1 = ld1; a.ld2 = ld2; a.ld3 = ld3; a.W1 = W1; a.W2 = W2; a.B = B;
@@ -407,6 +415,9 @@ extern "C" int svrs_elbo_bwd(const void* recon_x, const void* x, int dt_x, int d
     SVRS_CHECK_ARG(al16(d_recon_x) && al16(d_recon_y) && al16(d_mu1) && al16(d_lv1) && al16(d_mu2) && al16(d_lv2) && al16(d_mu3) && al16(d_lv3),
                    "elbo_bwd: gradient pointers must be 16B aligned");
     SVRS_CHECK_ARG(dld1 % 4 == 0 && dld2 % 4 == 0 && dld3 % 4 == 0, "elbo_bwd: gradient strides %% 4");
+    SVRS_CHECK_ARG(!mu1 || !(d_mu1 || d_lv1) || dld1 >= W1, "elbo_bwd: gradient row stride dld1 (%lld) < W1 (%d)", (long long)dld1, W1);
+    SVRS_CHECK_ARG(!mu2 || !(d_mu2 || d_lv2) || dld2 >= W2, "elbo_bwd: gradient row stride dld2 (%lld) < W2 (%d)", (long long)dld2, W2);
+    SVRS_CHECK_ARG(!mu2 || !(d_mu3 || d_lv3) || dld3 >= W2, "elbo_bwd: gradient row stride dld3 (%lld) < W2 (%d)", (long long)dld3, W2);
     a.drx = d_recon_x; a.dry = d_recon_y; a.dtdx = dt_dx; a.dtdy = dt_dy; a.act = act;
     a.dmu1 = d_mu1; a.dlv1 = d_lv1; a.dmu2 = d_mu2; a.dlv2 = d_lv2; a.dmu3 = d_mu3; a.dlv3 = d_lv3;
     a.dld1 = dld1; a.dld2 = dld2; a.dld3 = dld3;

@@ -234,6 +234,8 @@ extern "C" int svrs_sample_latents(const float* mu3, const float* lv3, int64_t l
                                    uint64_t sample_offset, const int64_t* step_ptr, void* stream) {
     SVRS_CHECK_ARG(mu3 && lv3 && yflat && stack, "sample_latents: null pointer");
     SVRS_CHECK_ARG(B > 0 && S > 0 && Wz > 0 && Wz % 4 == 0 && ld3 % 4 == 0 && ldy % 4 == 0, "sample_latents: B, S > 0 and Wz, ld3, ldy multiples of 4 required");
+    SVRS_CHECK_ARG(ld3 >= Wz && ldy >= Wz, "sample_latents: row strides ld3 (%lld) and ldy (%lld) must be >= Wz (%d)", (long long)ld3, (long long)ldy, Wz);
+    SVRS_CHECK_ARG(al16(mu3) && al16(lv3) && al16(yflat) && al16(eps) && al16(stack), "sample_latents: pointers must be 16B aligned");
     const long long nvec = (long long)B * S * (Wz / 4);
     const int blocks = (int)((nvec + 255) / 256 < (long long)num_sms() * 8 ? (nvec + 255) / 256 : (long long)num_sms() * 8);
     SVRS_LAUNCH(sample_latents_kernel, blocks, 256, 0, (cudaStream_t)stream, mu3, lv3, (long long)ld3, yflat, (long long)ldy, eps, stack,
@@ -260,6 +262,7 @@ extern "C" int svrs_sample_tail_stats(const void* x, int dtype, const void* w_kn
                                       float* sample0_nchw, void* stream) {
     SVRS_CHECK_ARG(x && w_kn && scratch, "sample_tail_stats: null pointer");
     SVRS_CHECK_ARG(dtype == SVRS_F32 || dtype == SVRS_BF16, "sample_tail_stats: bad dtype %d", dtype);
+    SVRS_CHECK_ARG(al16(x) && al16(target_nhwc), "sample_tail_stats: x and target_nhwc must be 16B aligned");
     SVRS_CHECK_ARG(B > 0 && S > 0 && H > 0 && W > 0, "sample_tail_stats: B, S, H, W must be positive");
     if (Cin != TS_CIN || Cout != TS_COUT) {
         set_error("sample_tail_stats: the fused tail is the 16 -> 4 conv of decoder_x (cond_vae.py:79); got %d -> %d", Cin, Cout);

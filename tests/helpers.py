@@ -39,6 +39,33 @@ def pack(w, dtype, convT=False):
     return (p01, p10) if convT else (p10, p01)
 
 
+class Guarded:
+    """A device tensor `t` of `shape` inside a buffer with `pad` sentinel elements before and after it: intact() is False
+    once a kernel has written outside `t`."""
+
+    SENTINEL = 12345.0
+
+    def __init__(self, shape, dtype, fill=float("nan"), pad=4096):
+        n = 1
+        for d in shape:
+            n *= int(d)
+        self.pad, self.n = pad, n
+        self.buf = torch.full((n + 2 * pad,), self.SENTINEL, device="cuda", dtype=dtype)
+        self.t = self.buf[pad:pad + n].view(shape)
+        self.t.fill_(fill)
+
+    def intact(self):
+        return bool((self.buf[:self.pad] == self.SENTINEL).all() and (self.buf[self.pad + self.n:] == self.SENTINEL).all())
+
+
+def task_stats(draws, target):
+    """models/base.py:305-313, 341 of the reference, verbatim arithmetic on a [S,4,P,P] sample stack and a [1,4,P,P] target."""
+    diff = draws - target
+    return dict(mean=draws.mean(dim=0), std=draws.std(dim=0).mean(dim=0), mae=diff.abs().mean(dim=(0, 1)),
+                mse=diff.pow(2).mean(dim=(0, 1)), mean_bias=(target - draws.mean(dim=0)).mean(dim=0).mean(dim=0),
+                sample0=draws[0])
+
+
 def report(name, got, ref, rtol, atol=0.0):
     got = got.detach().double().cpu()
     ref = ref.detach().double().cpu()

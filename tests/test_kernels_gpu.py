@@ -9,7 +9,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import BF16, F32, dt, lib, nchw, nhwc, pack, report, st
+from helpers import BF16, F32, Guarded, dt, lib, nchw, nhwc, pack, report, st
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -320,28 +320,62 @@ def test_philox_matches_numpy_restatement_and_is_normal():
 
 
 def test_reparam_fwd_bwd():
+    # ld_mult 2: z_ld = dz_ld = 2 Wd, z is the second half of the engine's torch.cat row; "nonzero": bwd accumulates, denc += ...
+    for ld_mult in (1, 2):
+        for denc0 in ("zero", "nonzero"):
+            _reparam_case(ld_mult, denc0)
+
+
+def _reparam_case(ld_mult, denc0):
     g = torch.Generator().manual_seed(8)
     B, Wd = 5, 256
+    ld = ld_mult * Wd
     enc = torch.randn(B, 2 * Wd, generator=g)
     eps = torch.randn(B, Wd, generator=g)
     er = enc.double().requires_grad_(True)
     zr = er[:, :Wd] + eps.double() * torch.exp(0.5 * er[:, Wd:])
     gz = torch.randn(B, Wd, generator=g)
     zr.backward(gz.double())
-    encd, epsd, gzd = enc.to(DEV), eps.to(DEV), gz.to(DEV)
-    z = torch.empty(B, Wd, device=DEV)
-    lib.reparam_fwd(encd.data_ptr(), epsd.data_ptr(), z.data_ptr(), Wd, None, B, Wd, 0, 0, 0, None, st())
-    report("reparam fwd", z, zr, 1e-6)
-    denc = torch.zeros(B, 2 * Wd, device=DEV)
-    lib.reparam_bwd(encd.data_ptr(), epsd.data_ptr(), gzd.data_ptr(), Wd, denc.data_ptr(), B, Wd, 0, 0, 0, None, st())
-    report("reparam bwd", denc, er.grad, 1e-6)
-    # on-device noise: eps_out replays exactly in backward
+    d0 = torch.zeros(B, 2 * Wd) if denc0 == "zero" else torch.randn(B, 2 * Wd, generator=g)
+    gzbuf = torch.full((B, ld), float("nan"))      # columns past Wd must not be read
+    gzbuf[:, :Wd] = gz
+    encd, epsd, gzd = enc.to(DEV), eps.to(DEV), gzbuf.to(DEV)
+    z = Guarded((B, ld), torch.float32)
+    lib.reparam_fwd(encd.data_ptr(), epsd.data_ptr(), z.t.data_ptr(), ld, None, B, Wd, 0, 0, 0, None, st())
+    report(f"reparam fwd [ld {ld}, denc {denc0}]", z.t[:, :Wd], zr, 1e-6)
+    assert torch.isnan(z.t[:, Wd:]).all() and z.intact(), "reparam_fwd wrote outside the first Wd columns of its rows"
+    denc = Guarded((B, 2 * Wd), torch.float32)
+    denc.t.copy_(d0)
+    lib.reparam_bwd(encd.data_ptr(), epsd.data_ptr(), gzd.data_ptr(), ld, denc.t.data_ptr(), B, Wd, 0, 0, 0, None, st())
+    report(f"reparam bwd [ld {ld}, denc {denc0}]", denc.t, d0.double() + er.grad, 1e-6)
+    assert denc.intact()
+    # on-device noise with a step counter: eps_out replays exactly in backward and is svrs_philox_normal's draw
+    step = torch.tensor([3], dtype=torch.int64, device=DEV)
     eo = torch.empty(B, Wd, device=DEV)
-    lib.reparam_fwd(encd.data_ptr(), None, z.data_ptr(), Wd, eo.data_ptr(), B, Wd, 77, 1, 3, None, st())
+    lib.reparam_fwd(encd.data_ptr(), None, z.t.data_ptr(), ld, eo.data_ptr(), B, Wd, 77, 1, 3, step.data_ptr(), st())
+    ref_eps = torch.empty(B, Wd, device=DEV)
+    lib.philox_normal(ref_eps.data_ptr(), B, Wd, 77, 1, 3, step.data_ptr(), st())
+    assert torch.equal(eo, ref_eps)
     d1 = torch.zeros(B, 2 * Wd, device=DEV); d2 = torch.zeros(B, 2 * Wd, device=DEV)
-    lib.reparam_bwd(encd.data_ptr(), None, gzd.data_ptr(), Wd, d1.data_ptr(), B, Wd, 77, 1, 3, None, st())
-    lib.reparam_bwd(encd.data_ptr(), eo.data_ptr(), gzd.data_ptr(), Wd, d2.data_ptr(), B, Wd, 77, 1, 3, None, st())
+    lib.reparam_bwd(encd.data_ptr(), None, gzd.data_ptr(), ld, d1.data_ptr(), B, Wd, 77, 1, 3, step.data_ptr(), st())
+    lib.reparam_bwd(encd.data_ptr(), eo.data_ptr(), gzd.data_ptr(), ld, d2.data_ptr(), B, Wd, 77, 1, 3, step.data_ptr(), st())
     assert torch.equal(d1, d2)
+    eo4 = torch.empty(B, Wd, device=DEV)
+    step4 = torch.tensor([4], dtype=torch.int64, device=DEV)
+    lib.reparam_fwd(encd.data_ptr(), None, z.t.data_ptr(), ld, eo4.data_ptr(), B, Wd, 77, 1, 3, step4.data_ptr(), st())
+    assert float((eo4 == eo).double().mean()) < 1e-3, "another step gave the same noise"
+    # partition invariance: rows [2, 5) drawn alone at sample_offset 3 + 2 equal rows 2..4 of the full draw
+    zp = Guarded((3, ld), torch.float32)
+    ep = torch.empty(3, Wd, device=DEV)
+    lib.reparam_fwd(encd.data_ptr() + 4 * 2 * 2 * Wd, None, zp.t.data_ptr(), ld, ep.data_ptr(), 3, Wd, 77, 1, 3 + 2, step.data_ptr(), st())
+    lib.reparam_fwd(encd.data_ptr(), None, z.t.data_ptr(), ld, eo.data_ptr(), B, Wd, 77, 1, 3, step.data_ptr(), st())
+    assert torch.equal(ep, eo[2:]) and torch.equal(zp.t[:, :Wd], z.t[2:, :Wd]) and zp.intact()
+    # B = 0 enqueues nothing
+    torch.cuda.synchronize()
+    n0, before = lib.launch_count(), denc.t.clone()
+    lib.reparam_fwd(encd.data_ptr(), None, z.t.data_ptr(), ld, None, 0, Wd, 77, 1, 3, step.data_ptr(), st())
+    lib.reparam_bwd(encd.data_ptr(), None, gzd.data_ptr(), ld, denc.t.data_ptr(), 0, Wd, 77, 1, 3, step.data_ptr(), st())
+    assert lib.launch_count() == n0 and torch.equal(denc.t, before)
 
 
 def test_elbo_against_golden_vectors(golden_dir):

@@ -11,7 +11,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import BF16, F32, dt, lib, nchw, nhwc, pack, report, st
+from helpers import BF16, F32, Guarded, dt, lib, nchw, nhwc, pack, report, st, task_stats
 from oracle import ref_oracle as O
 from svrs_native.lib import SvrsUnsupported
 
@@ -276,14 +276,6 @@ def test_adam_multi_direct(grad_layout):
 
 
 # ------------------------------------------------------------------------------------------------ f4: fused uncertainty maps
-def _task_stats(draws, target):
-    """models/base.py:305-313, 341 of the reference, verbatim arithmetic on a [S,4,P,P] sample stack."""
-    diff = draws - target
-    return dict(mean=draws.mean(dim=0), std=draws.std(dim=0).mean(dim=0), mae=diff.abs().mean(dim=(0, 1)),
-                mse=diff.pow(2).mean(dim=(0, 1)), mean_bias=(target - draws.mean(dim=0)).mean(dim=0).mean(dim=0),
-                sample0=draws[0])
-
-
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 def test_sample_stats_fused_tail_matches_reference_statistics(golden_dir, dtype):
     """Streaming Welford statistics in the decoder tail (svrs_sample_tail_stats) == the reference's statistics of the
@@ -299,10 +291,10 @@ def test_sample_stats_fused_tail_matches_reference_statistics(golden_dir, dtype)
     eu, es = r.randn(1, eng.Wu), r.randn(S, eng.Wz)
     x, y = FX.inputs(fx)
     y1, x1 = y[1:2], x[1:2]
-    ref = _task_stats(O.cond_sample({k: v.clone() for k, v in sd.items()}, 2, 64, y1, eu, es, training=False).double(), x1.double())
+    ref = task_stats(O.cond_sample({k: v.clone() for k, v in sd.items()}, 2, 64, y1, eu, es, training=False).double(), x1.double())
     tol = 2e-5 if dtype == torch.float32 else 2e-2
     with torch.no_grad():
-        own = _task_stats(model.sample(y1.to(DEV), samples=S, eps_u=eu.to(DEV), eps_s=es.to(DEV)).double(), x1.to(DEV).double())
+        own = task_stats(model.sample(y1.to(DEV), samples=S, eps_u=eu.to(DEV), eps_s=es.to(DEV)).double(), x1.to(DEV).double())
         for splits in (1, 3, 4, 0):
             st = model.sample_stats(y1.to(DEV), samples=S, target=x1.to(DEV), eps_u=eu.to(DEV), eps_s=es.to(DEV), splits=splits)
             for k in ("mean", "std", "mae", "mse", "mean_bias", "sample0"):
@@ -341,18 +333,6 @@ def test_sample_stats_batched_patches_match_single(golden_dir):
 # ------------------------------------------------------------------------------------------------ narrow layers: guard bands
 # (compute-sanitizer is closed on the GPU pool: out-of-bounds WRITES are caught with sentinel guard bands around every output,
 # partial 16-pixel steps and non-power-of-two maps exercise the tail / division paths of the mma.sync narrow kernels)
-class _Guarded:
-    def __init__(self, shape, dtype, fill=float("nan"), pad=4096):
-        n = int(np.prod(shape))
-        self.pad, self.n = pad, n
-        self.buf = torch.full((n + 2 * pad,), 12345.0, device=DEV, dtype=dtype)
-        self.t = self.buf[pad:pad + n].view(shape)
-        self.t.fill_(fill)
-
-    def intact(self):
-        return bool((self.buf[:self.pad] == 12345.0).all() and (self.buf[self.pad + self.n:] == 12345.0).all())
-
-
 @pytest.mark.parametrize("case", [(3, 12, 20, 4, 4, 3), (3, 12, 20, 16, 4, 3), (2, 20, 12, 4, 16, 3), (5, 6, 6, 4, 16, 4), (1, 64, 64, 16, 4, 3),
                                   (2, 10, 6, 4, 4, 4), (7, 4, 4, 16, 4, 4),
                                   # 16 / 64 -> 16 channels: wgrad16 (mma.sync + ldmatrix.trans from staged rows)
@@ -372,10 +352,10 @@ def test_narrow_mma_kernels_odd_shapes_and_guard_bands(case):
     OH, OW = yr.shape[2:]
     xd, wd, bd, gyd = nhwc(x.to(DEV), torch.bfloat16), w.to(DEV), b.to(DEV), nhwc(gy.to(DEV), torch.bfloat16)
     pf, pb = pack(wd, torch.bfloat16)
-    y = _Guarded((N, OH, OW, Cout), torch.bfloat16)
-    dx = _Guarded((N, H, W, Cin), torch.bfloat16)
-    dw = _Guarded((Cout, Cin, ks, ks), torch.float32, fill=0.0)
-    db = _Guarded((Cout,), torch.float32, fill=0.0)
+    y = Guarded((N, OH, OW, Cout), torch.bfloat16)
+    dx = Guarded((N, H, W, Cin), torch.bfloat16)
+    dw = Guarded((Cout, Cin, ks, ks), torch.float32, fill=0.0)
+    db = Guarded((Cout,), torch.float32, fill=0.0)
     lib.conv2d_fprop(xd.data_ptr(), pf.data_ptr(), pb.data_ptr(), bd.data_ptr(), y.t.data_ptr(), BF16, N, H, W, Cin, Cout, ks, 0, st())
     lib.conv2d_dgrad(gyd.data_ptr(), pb.data_ptr(), pf.data_ptr(), dx.t.data_ptr(), BF16, N, H, W, Cin, Cout, ks, st())
     lib.conv2d_wgrad(xd.data_ptr(), gyd.data_ptr(), dw.t.data_ptr(), None, db.t.data_ptr(), BF16, N, H, W, Cin, Cout, ks, 0, st())
