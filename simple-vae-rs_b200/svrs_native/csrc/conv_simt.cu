@@ -314,7 +314,6 @@ struct WgradArgs {
 
 }  // namespace svrs
 #include "wgrad_narrow.cuh"   // bf16 narrow weight gradients on mma.sync + movmatrix (needs WgradArgs)
-#include "wgrad16.cuh"        // 16 / 64 -> 16 channel 3x3 weight gradients on mma.sync + ldmatrix.trans
 namespace svrs {
 
 template <typename T>
@@ -922,10 +921,7 @@ extern "C" int svrs_conv2d_wgrad(const void* x, const void* dy, float* dw, float
         else geom_conv4s2(a.g, N, H, W, Cin, Cout);
         // the tensor-core kernels fold the bias gradient (column sums of dy) into their idle epilogue warps
         const bool fold_db = db != nullptr && Cout % 8 == 0;
-        if (g_tc_enabled_narrow && ksplit <= 0 && wgrad16_takes(dtype, N, H, W, Cin, Cout, ksize)) {
-            rc = launch_wgrad16(x, dy, dw, db, N, H, W, Cin, (cudaStream_t)stream);      // torch layout, bias folded in
-            db = nullptr;
-        } else if (g_tc_enabled && N > 0 && dtype == SVRS_BF16 && wgrad_halo_supported(a.g, a.KK)) {
+        if (g_tc_enabled && N > 0 && dtype == SVRS_BF16 && wgrad_halo_supported(a.g, a.KK)) {
             rc = launch_wgrad3_halo(a.g, dy, x, dw_packed ? dw_packed : dw, dw_packed != nullptr, fold_db ? db : nullptr, (cudaStream_t)stream);
             if (fold_db) db = nullptr;
         } else if (g_tc_enabled && N > 0 && wgrad_tc_supported(dtype, Cout, Cin, a.g.OW, a.g.OH)) {
@@ -969,7 +965,6 @@ extern "C" int svrs_convT2d_wgrad(const void* x, const void* dy, float* dw, floa
 // (Same decision tree as svrs_conv2d_wgrad / svrs_convT2d_wgrad; the fused optimiser reads the gradient accordingly.)
 extern "C" int svrs_conv2d_wgrad_layout(int dtype, int N, int H, int W, int Cin, int Cout, int ksize) {
     if (!(ksize == 3 || (ksize == 4 && H % 2 == 0 && W % 2 == 0)) || N <= 0) return 0;
-    if (g_tc_enabled_narrow && wgrad16_takes(dtype, N, H, W, Cin, Cout, ksize)) return 0;
     TapGeom g;
     if (ksize == 3) geom_conv3(g, N, H, W, Cin, Cout, false);
     else geom_conv4s2(g, N, H, W, Cin, Cout);

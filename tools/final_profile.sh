@@ -24,7 +24,6 @@ cap wgrad_tc_kernel 8 wgrad_tc
 cap conv3_halo_kernel 6 conv3_halo
 cap convT_halo_kernel 3 convT_halo
 cap wgrad3_halo_kernel 4 wgrad3_halo
-cap wgrad16_mma_kernel 2 wgrad16
 cap adam_multi_kernel 1 adam_multi
 cap "bn_" 6 bn
 cap "elbo_|reparam_|patch_tma" 6 elbo_reparam_patch
