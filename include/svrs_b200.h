@@ -75,9 +75,10 @@ int svrs_pack_weights_multi(const void* jobs, int njobs, int total_tiles, int ma
 int svrs_unpack_grads_multi(const void* jobs, int njobs, int total_tiles, int max_kk, void* stream);
 
 /* Two kernels sit behind each fprop/dgrad entry point:
- *   - conv_tc   (csrc/conv_tc.cu): tcgen05.mma + TMEM accumulators + TMA-fed SWIZZLE_128B operands; taken when
- *     dtype == BF16, the reduction channels are a multiple of 64, the written channels a multiple of 16 and the
- *     output map tiles into 128-pixel boxes; it consumes the NK pack `w_nk` = [tap][N][K] (K contiguous).
+ *   - conv_tc   (csrc/conv_tc.cu): tcgen05.mma + TMEM accumulators + TMA-fed swizzled operands; taken when
+ *     dtype == BF16, the reduction channels K are a multiple of 8 and at least 16 (16-byte NHWC rows; when K % 16 != 0
+ *     the last 64-channel chunk is TMA zero fill past K), the written channels a multiple of 4 and the output map tiles
+ *     into 128-pixel boxes; it consumes the NK pack `w_nk` = [tap][N][K] (K contiguous).
  *   - conv_simt (csrc/conv_simt.cu): fp32-FMA multi-tap GEMM for everything else (fp32 parity mode, 4/16-channel
  *     layers, odd channel counts); it consumes the KN pack `w_kn` = [tap][K][N].
  * The two packs of a layer are each other's transposes, i.e. the (p01, p10) pair of svrs_pack_weights: the KN pack
@@ -86,7 +87,10 @@ void svrs_set_tc_enabled(int enabled);   /* default 1; 0 forces the SIMT kernels
 /* conv3_halo (csrc/conv_halo.cu): 3x3 stride-1 fprop/dgrad on maps tiling into 8x16 blocks load each tile's activation
  * halo ONCE and address the nine taps as shared-memory descriptors.  mode 0 = off (per-tap TMA kernel), 1 = on (default). */
 void svrs_set_halo_mode(int mode);
-int svrs_tc_would_run(int dtype, int K, int Nc, int OH, int OW); /* 1 if conv_tc takes a GEMM of these dims */
+/* 1 if conv_tc takes a GEMM of these dims.  Channel rule of the tcgen05 kernels (conv_tc and the wgrad kernels below):
+ * C % 8 == 0 and C >= 16 for the channels a kernel reads through TMA; channel counts with rows that are not 16-byte
+ * multiples (42, 84, 53, 106, 212, ...) and 8-channel operands go to the CUDA-core kernels. */
+int svrs_tc_would_run(int dtype, int K, int Nc, int OH, int OW);
 
 /* ---- nn.Conv2d k3 s1 p1 / k4 s2 p1 (layers.py:231-236; every bare nn.Conv2d of cond_vae.py / vae.py)
  *      x [N,H,W,Cin] -> y [N,H/s,W/s,Cout];  w_kn = p10 pack [tap][Cin][Cout]; bias fp32 [Cout] or NULL.
@@ -140,7 +144,9 @@ int svrs_convT2d_dgrad(const void* dy, const void* w_kn, const void* w_nk, void*
 int svrs_convT2d_wgrad(const void* x, const void* dy, float* dw, float* dw_packed, float* db, int dtype,
                        int N, int H, int W, int Cin, int Cout, int ksplit, void* stream);
 
-/* Layout the wgrad entry points leave in dw_packed for a problem: 1 = per-tap packed [tap][d1][d0] (tcgen05 kernels),
+/* Layout the wgrad entry points leave in dw_packed for a problem: 1 = per-tap packed [tap][d1][d0] (tcgen05 kernels:
+ * bf16 with both channel counts multiples of 8 and at least 16, the channel rule of svrs_tc_would_run, and a map that
+ * tiles into 128-pixel boxes; ragged boxes are zero-filled and clipped, nothing outside [kk][d1][d0] is written),
  * 0 = nothing (a SIMT kernel accumulates torch layout into dw).  The fused optimiser (svrs_adam_multi) passes the SAME
  * buffer as dw and dw_packed and reads the gradient in whichever layout this reports, so no unpack pass is needed. */
 int svrs_conv2d_wgrad_layout(int dtype, int N, int H, int W, int Cin, int Cout, int ksize);

@@ -14,6 +14,9 @@
 //     in the matching SWIZZLE_128B / 64B / 32B K-major layout (8-row groups 1024 / 512 / 256 B apart), consumed
 //     directly by tcgen05.mma (M=128, N=n_tile, K=16) through shared-memory descriptors.  For cw < 64 a pipeline
 //     stage carries 64/cw (tap, chunk) pairs so a stage always moves ~16 KB of activations.
+//     Reduction channels that are a multiple of 8 but not of 16 (16-byte rows, e.g. 168 / 424) take ceil(K / cw) chunks
+//     of cw = 64 (or the narrowest of 16 / 32 / 64 covering K <= 64): both tensor maps keep the true K as their inner
+//     dimension, so the channels past K in the last box arrive as TMA zero fill in A and B and add nothing.
 //   * accumulators live in TMEM (2 stages x 256 columns) so the epilogue of tile i overlaps the
 //     main loop of tile i+1; the epilogue (4 warps) does tcgen05.ld -> +bias -> activation -> bf16 ->
 //     128-bit global stores, one output pixel (row) per thread.  Output channels are padded to a multiple of 16
@@ -243,7 +246,15 @@ static CUtensorMapSwizzle swizzle_for(int cw) {
     return cw == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (cw == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
 }
 
-int chunk_width(int C) { return C % 64 == 0 ? 64 : (C % 32 == 0 ? 32 : (C % 16 == 0 ? 16 : 0)); }
+// Channel chunk of a tcgen05 operand with C channels: the widest of 64 / 32 / 16 dividing C; for C % 16 != 0 with 16-byte
+// rows (C % 8 == 0) the last chunk is ragged: 64 when C > 64, otherwise the narrowest width covering C.  0 = unsupported:
+// rows that are not 16-byte multiples (no TMA map describes them), and C = 8, which would fill half of every MMA with zero
+// fill - 8-channel operands stay on the CUDA-core kernels, no measurement shows the tensor cores winning there.
+int chunk_width(int C) {
+    if (C % 16 == 0) return C % 64 == 0 ? 64 : (C % 32 == 0 ? 32 : 16);
+    if (C % 8 != 0 || C < 24) return 0;
+    return C > 32 ? 64 : (C > 16 ? 32 : 16);
+}
 
 // 4-D activation view map: dims (C, W, H, N) with arbitrary element strides for W/H/N; box (cw, BW, BH, BNI)
 int make_act_map(CUtensorMap* m, const void* base, int C, int W, int H, int N, long long sx, long long sy, long long sn,
@@ -272,6 +283,22 @@ int make_f32_2d_map(CUtensorMap* m, const void* base, long long inner, long long
     CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides, box, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(f32 2d) failed: %d (inner=%lld rows=%lld box %dx%d)", (int)r, inner, rows, box_inner, box_rows); return SVRS_E_CUDA; }
+    return 0;
+}
+
+// fp32 [d2][d1][d0] (d0 contiguous), box (box0 = 32 or 16 columns, box1 rows, 1): the per-tap packed gradient seen with its
+// true extents, so a box that reaches past d0 or d1 is clipped by TMA instead of spilling into the next tap
+int make_f32_3d_map(CUtensorMap* m, const void* base, long long d0, long long d1, long long d2, int box0, int box1) {
+    PFN_encodeTiled enc = get_encode();
+    if (!enc) { set_error("cuTensorMapEncodeTiled unavailable"); return SVRS_E_CUDA; }
+    cuuint64_t dims[3] = {(cuuint64_t)d0, (cuuint64_t)d1, (cuuint64_t)d2};
+    cuuint64_t strides[2] = {(cuuint64_t)d0 * 4, (cuuint64_t)(d0 * d1) * 4};
+    cuuint32_t box[3] = {(cuuint32_t)box0, (cuuint32_t)box1, 1};
+    cuuint32_t es[3] = {1, 1, 1};
+    CUtensorMapSwizzle sw = box0 * 4 == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, es,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(f32 3d) failed: %d (%lld x %lld x %lld box %dx%d)", (int)r, d0, d1, d2, box0, box1); return SVRS_E_CUDA; }
     return 0;
 }
 
@@ -327,7 +354,8 @@ bool pick_box(int OW, int OH, int& BW, int& BH, int& BNI) {
 
 bool tc_supported(int dtype, int K, int Nc, int OW, int OH) {
     int bw, bh, bn;
-    // K % 16: UMMA K; Nc % 4: 8-byte aligned output rows (N is padded to 16 for the MMA); K*2 B rows must be 16-B multiples
+    // K % 8: 16-byte rows for the TMA maps (a ragged last chunk is zero-filled up to the UMMA K of 16, see chunk_width);
+    // Nc % 4: 8-byte aligned output rows (N is padded to 16 for the MMA)
     return dtype == SVRS_BF16 && chunk_width(K) != 0 && Nc % 4 == 0 && Nc >= 4 && pick_box(OW, OH, bw, bh, bn);
 }
 
@@ -381,7 +409,7 @@ int launch_conv_tc(int form, const void* in, const void* w_nk, const float* bias
     p.n_tiles = (Cw + p.n_tile - 1) / p.n_tile;
     p.cw = chunk_width(Cr);
     p.tg = 64 / p.cw;
-    p.kchunks = Cr / p.cw;
+    p.kchunks = (Cr + p.cw - 1) / p.cw;      // the last chunk may be ragged: TMA zero-fills its channels past Cr
     p.act = act; p.nprob = g.nprob;
 
     // input maps: distinct in_off values become distinct tensor maps (parity classes of a stride-2 read)

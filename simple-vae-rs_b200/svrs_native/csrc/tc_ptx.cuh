@@ -48,6 +48,11 @@ __device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* map, uint32
                  ::"l"(map), "r"(src), "r"(c0), "r"(c1)
                  : "memory");
 }
+__device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
+    asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];"
+                 ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2)
+                 : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
@@ -377,6 +382,8 @@ int make_act_map(CUtensorMap* m, const void* base, int C, int W, int H, int N, l
 bool pick_box(int OW, int OH, int& BW, int& BH, int& BNI);
 // fp32 matrix [rows][inner] (inner contiguous), box (box_inner = 32 or 16 columns, box_rows), swizzle matching the box width
 int make_f32_2d_map(CUtensorMap* m, const void* base, long long inner, long long rows, int box_inner, int box_rows);
-int chunk_width(int C);   // 64 / 32 / 16 / 0 (unsupported)
+// fp32 [d2][d1][d0] (d0 contiguous), box (box0 = 32 or 16 columns, box1 rows, 1), OOB parts of a box are clipped
+int make_f32_3d_map(CUtensorMap* m, const void* base, long long d0, long long d1, long long d2, int box0, int box1);
+int chunk_width(int C);   // 64 / 32 / 16 (last chunk ragged when C % 16 != 0) / 0 (C % 8 != 0 or C == 8: unsupported)
 
 }  // namespace svrs

@@ -10,7 +10,9 @@
 //   * K = 128 pixels per pipeline stage (8 MMAs of K=16); the pixel range is split over CTAs.
 //   * every CTA keeps up to 512/N M-blocks of accumulators resident in TMEM for its whole pixel range and
 //     finishes with fp32 atomics into the torch-layout gradient dw[(a*Cb + b)*KK + tap].
-// TMA zero-fill implements the convolution padding for X and masks out-of-range images for G.
+// TMA zero-fill implements the convolution padding for X and masks out-of-range images for G.  It also pads ragged channel
+// counts (Ca or Cb % 8 == 0 but not a multiple of the box width): the last G / X box reads zeros past Ca / Cb, so those
+// accumulator columns / rows are zero, and the epilogues clip them (3-D reduce map, masked atomics, masked bias sums).
 #include "common.cuh"
 #include "taps.cuh"
 #include "tc_ptx.cuh"
@@ -35,7 +37,7 @@ struct WgTap { int map, dy, dx, tapid; };
 struct alignas(64) WgParams {
     CUtensorMap x_maps[4];    // input views (parity classes)
     CUtensorMap g_map;        // output-grid operand
-    CUtensorMap dw_map;       // packed mode: fp32 scratch [KK*Cb rows][Ca], box (min(32, n_tile) columns, cwx rows)
+    CUtensorMap dw_map;       // packed mode: fp32 scratch [KK][Cb][Ca], box (min(32, n_tile) columns, cwx rows, 1 tap)
     float* dw;
     float* db;                         // != NULL: bias gradient (column sums of G) folded in, see colsum_tile8
     const __nv_bfloat16* gptr;         // G base (output view) and its element strides, for the folded column sums
@@ -45,7 +47,7 @@ struct alignas(64) WgParams {
     int Ca, Cb, KK;
     int n_tile, n_tiles;               // columns (a) per CTA
     int cwx, cwg;                      // box widths (channels) of the X and G operands
-    int cb_chunks;                     // Cb / cwx
+    int cb_chunks;                     // ceil(Cb / cwx)
     int bpb;                           // boxes per M-block = 128 / cwx
     int nboxes, nblocks, group, ngroups;
     int ksplit, ksteps_total;
@@ -173,7 +175,9 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_tc_kernel(const __grid_co
             const int cg = p.n_tile / 8, lanes = 128 / cg;
             const int t = threadIdx.x - 64, cq = t % cg, cl = t / cg;
             float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-            for (int kstep = k_begin + grp; kstep < k_end; kstep += p.ngroups) {
+            // Ca % 8 == 0: an 8-column group lies wholly inside or wholly past the last G column (ragged last tile)
+            const int kfirst = nt * p.n_tile + cq * 8 < p.Ca ? k_begin + grp : k_end;
+            for (int kstep = kfirst; kstep < k_end; kstep += p.ngroups) {
                 int pt = kstep;
                 const int tx = pt % p.tiles_x; pt /= p.tiles_x;
                 const int ty = pt % p.tiles_y;
@@ -217,9 +221,9 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_tc_kernel(const __grid_co
                     for (int hh = 0; hh < p.bpb; ++hh) {
                         const int box = p.bpb * (blk0 + b) + hh;
                         if (box >= p.nboxes) break;                       // tail rows of the last M-block
-                        const int row0 = p.taps[box / p.cb_chunks].tapid * p.Cb + (box % p.cb_chunks) * p.cwx;
-                        for (int cc = 0; cc < nch; ++cc)
-                            tma_reduce_add_2d(&p.dw_map, buf + (uint32_t)(hh * nch + cc) * box_bytes, nt * p.n_tile + cc * cwd, row0);
+                        const int tapid = p.taps[box / p.cb_chunks].tapid, row0 = (box % p.cb_chunks) * p.cwx;
+                        for (int cc = 0; cc < nch; ++cc)      // the map clips columns >= Ca and rows >= Cb of a ragged box
+                            tma_reduce_add_3d(&p.dw_map, buf + (uint32_t)(hh * nch + cc) * box_bytes, nt * p.n_tile + cc * cwd, row0, tapid);
                     }
                     bulk_commit();
                 }
@@ -228,10 +232,10 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_tc_kernel(const __grid_co
         } else {
             for (int b = 0; b < nblk; ++b) {
                 const int box = p.bpb * (blk0 + b) + m / p.cwx;
-                const bool row_ok = box < p.nboxes;
-                const int bx = row_ok ? box : 0;
+                const int bx = box < p.nboxes ? box : 0;
                 const int tapid = p.taps[bx / p.cb_chunks].tapid;
                 const int cb = (bx % p.cb_chunks) * p.cwx + (m % p.cwx);
+                const bool row_ok = box < p.nboxes && cb < p.Cb;         // rows past Cb: zero fill of a ragged X box
                 const uint32_t taddr = tmem_base + (uint32_t)(b * p.n_tile) + ((uint32_t)(q * 32) << 16);
                 for (int c0 = 0; c0 < p.n_tile; c0 += 32) {
                     uint32_t v[32];
@@ -286,9 +290,9 @@ static void wg_prof_report(const WgParams& p, int grid, long long* dprof) {
 
 bool wgrad_tc_supported(int dtype, int Ca, int Cb, int OW, int OH) {
     int bw, bh, bn;
-    // Ca: 16 / 32 (single narrow box) or a multiple of 64 ; Cb: any multiple of 16
-    const bool ca_ok = Ca == 16 || Ca == 32 || (Ca >= 64 && Ca % 64 == 0);
-    return dtype == SVRS_BF16 && ca_ok && chunk_width(Cb) != 0 && pick_box(OW, OH, bw, bh, bn);
+    // Ca, Cb: multiples of 8 (16-byte rows for the TMA maps), at least 16 (see chunk_width); G / X boxes past Ca / Cb are
+    // zero-filled (see wg_plan)
+    return dtype == SVRS_BF16 && Ca >= 16 && Ca % 8 == 0 && chunk_width(Cb) != 0 && pick_box(OW, OH, bw, bh, bn);
 }
 
 // Tiling / split plan of one launch (everything except the tensor maps).  The pixel split is exact - every split owns at
@@ -299,11 +303,13 @@ static int wg_plan(const TapGeom& g, int KK, WgParams& p) {
     p.N = g.N; p.OH = g.OH; p.OW = g.OW;
     p.tiles_x = g.OW / p.BW; p.tiles_y = g.OH / p.BH; p.tiles_n = (g.N + p.BNI - 1) / p.BNI;
     p.Ca = g.Nc; p.Cb = g.K; p.KK = KK;
-    p.n_tile = p.Ca < 128 ? p.Ca : 128;
+    // G boxes: one box of 16 / 32 / 64 columns covering Ca <= 64, otherwise 128-column tiles of two 64-column boxes.  Ca = 16,
+    // 32 and multiples of 64 fill their boxes; other multiples of 8 leave zero-filled columns in the last box.
+    p.cwg = p.Ca <= 16 ? 16 : (p.Ca <= 32 ? 32 : 64);
+    p.n_tile = p.Ca <= 64 ? p.cwg : 128;
     p.n_tiles = (p.Ca + p.n_tile - 1) / p.n_tile;
-    p.cwg = p.Ca < 64 ? p.Ca : 64;
     p.cwx = chunk_width(p.Cb);
-    p.cb_chunks = p.Cb / p.cwx;
+    p.cb_chunks = (p.Cb + p.cwx - 1) / p.cwx;
     p.bpb = 128 / p.cwx;
     const Prob& pb = g.prob[0];
     p.ntaps = pb.ntaps;
@@ -380,7 +386,7 @@ int launch_wgrad_tc(const TapGeom& g, const void* gmat, const void* x, float* dw
     if (rc) return rc;
 
     if (packed) {
-        rc = make_f32_2d_map(&p.dw_map, dw, p.Ca, (long long)KK * p.Cb, p.n_tile < 32 ? p.n_tile : 32, p.cwx);
+        rc = make_f32_3d_map(&p.dw_map, dw, p.Ca, p.Cb, KK, p.n_tile < 32 ? p.n_tile : 32, p.cwx);
         if (rc) return rc;
     }
 
